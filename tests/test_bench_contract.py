@@ -36,6 +36,32 @@ def test_committed_b200_record_has_contract_keys():
     assert d["metric"].startswith("Lurk iterations proved/sec") and d["config"]["workload"]
 
 
+def test_dump_outputs_writes_exact_float64_limbs(tmp_path):
+    """--dump-outputs: every field element becomes eight exact 32-bit limbs in float64; long W / E keep a seeded sample of rows"""
+    import numpy as np
+    from types import SimpleNamespace
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(3)
+    elems = lambda n: rng.integers(0, 256, size=n * 32, dtype=np.uint8)
+    rec = SimpleNamespace(comm_W=elems(3), comm_T=elems(3), r=elems(1), running_comm_W=elems(3), running_comm_E=elems(3), ro_hash=elems(1))
+    run = dict(W=elems(100), E=elems(30), u=elems(1), X=elems(2))
+    ctx = SimpleNamespace(get_running=lambda: run)
+    wl = SimpleNamespace(names=["primary"], inst=[SimpleNamespace(ctx=ctx)], last=[rec])
+    for out in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(wl, str(out), sample=40)
+    to_bytes = lambda a: a.astype("<u4").tobytes()
+    for k in ("comm_W", "comm_T", "r", "running_comm_W", "running_comm_E", "ro_hash"):
+        a = np.load(tmp_path / "a" / f"primary_{k}.npy")
+        assert a.dtype == np.float64 and a.shape[1] == 8 and to_bytes(a) == getattr(rec, k).tobytes()
+    assert to_bytes(np.load(tmp_path / "a" / "primary_running_E.npy")) == run["E"].tobytes()
+    assert to_bytes(np.load(tmp_path / "a" / "primary_running_X.npy")) == run["X"].tobytes()
+    w = np.load(tmp_path / "a" / "primary_running_W.npy")
+    assert w.shape == (40, 8) and np.array_equal(w, np.load(tmp_path / "b" / "primary_running_W.npy"))
+    rows = {to_bytes(w[i:i + 1]) for i in range(40)}
+    assert len(rows) == 40 and rows <= {run["W"][32 * i:32 * i + 32].tobytes() for i in range(100)}
+
+
 def test_synthetic_step_circuit_is_satisfiable_by_construction():
     """bench.py's full-size R1CS generator (vectorised) obeys the rule it documents: with the glue columns defined by the
     product rows, any slot-column content satisfies (A z) o (B z) = (C z); checked on the oracle at a small size"""
