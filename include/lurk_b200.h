@@ -247,6 +247,12 @@ int lurk_sumcheck_prove_batch_dev(int field_id, int kind, int n_instances, void 
 int lurk_eq_evals_dev(int field_id, const uint8_t *tau, int num_vars, void *d_out, int fmt, void *stream);
 /* <a, b> over n Montgomery elements (MultilinearPolynomial::evaluate = <Z, eq(r)>; the c_L / c_R of an IPA round).  Synchronous. */
 int lurk_inner_product_dev(int field_id, const void *d_a, const void *d_b, size_t n, uint8_t out[32], int fmt, void *stream);
+/* PolyEvalWitness::batch_diff_size (batch_eval_reduce's joint polynomial): d_out[i] = sum_{j : i < lens[j]} coeffs[j] * P_j[i] for
+ * i < out_len, zero where no P_j reaches -- every P_j zero-extended at the end.  n_polys <= 120 device polynomials of lens[j] <= out_len
+ * Montgomery elements (d_polys / lens / coeffs: host arrays; coeffs: n_polys x 32 bytes in `fmt`).  d_out must not overlap any P_j.
+ * One launch; asynchronous on `stream`. */
+int lurk_poly_combine_dev(int field_id, int n_polys, const void *const *d_polys, const size_t *lens, const uint8_t *coeffs, void *d_out,
+                          size_t out_len, int fmt, void *stream);
 /* one IPA folding step, in place on the first n / 2 slots: a[i] <- x a[i] + y a[i + n/2];  G[i] <- x G[i] + y G[i + n/2]
  * (CommitmentKey::fold; bases affine Montgomery; x, y host scalars in `fmt`). */
 int lurk_ipa_fold_scalars_dev(int field_id, void *d_a, size_t n, const uint8_t x[32], const uint8_t y[32], int fmt, void *stream);

@@ -89,6 +89,8 @@ extern "C" {
                                    user: *mut c_void, round_evals: *mut u8, challenges: *mut u8, final_evals: *mut u8, fmt: c_int, stream: *mut c_void) -> c_int;
     pub fn lurk_eq_evals_dev(field_id: c_int, tau: *const u8, num_vars: c_int, d_out: *mut c_void, fmt: c_int, stream: *mut c_void) -> c_int;
     pub fn lurk_inner_product_dev(field_id: c_int, d_a: *const c_void, d_b: *const c_void, n: usize, out: *mut u8, fmt: c_int, stream: *mut c_void) -> c_int;
+    pub fn lurk_poly_combine_dev(field_id: c_int, n_polys: c_int, d_polys: *const *const c_void, lens: *const usize, coeffs: *const u8, d_out: *mut c_void,
+                                 out_len: usize, fmt: c_int, stream: *mut c_void) -> c_int;
     pub fn lurk_ipa_prove_dev(curve_id: c_int, ck: *mut lurk_msm_ctx, ck_c: *const u8, d_a: *mut c_void, d_b: *mut c_void, log_n: c_int, challenge: lurk_challenge_fn,
                               user: *mut c_void, l_out: *mut u8, r_out: *mut u8, a_final: *mut u8, b_final: *mut u8, fmt: c_int, stream: *mut c_void) -> c_int;
     pub fn lurk_hyperkzg_prove_dev(curve_id: c_int, ck: *mut lurk_msm_ctx, d_poly: *const c_void, point: *const u8, num_vars: c_int, challenge: lurk_challenge_fn,

@@ -95,6 +95,7 @@ PROTOTYPES = {
     "lurk_sumcheck_prove_batch_dev": (_i, [_i, _i, _i, C.POINTER(_vp), C.POINTER(_i), _vp, _vp, CHALLENGE_FN, _vp, _vp, _vp, _vp, _i, _vp]),
     "lurk_eq_evals_dev": (_i, [_i, _vp, _i, _vp, _i, _vp]),
     "lurk_inner_product_dev": (_i, [_i, _vp, _vp, _sz, _vp, _i, _vp]),
+    "lurk_poly_combine_dev": (_i, [_i, _i, C.POINTER(_vp), C.POINTER(_sz), _vp, _vp, _sz, _i, _vp]),
     "lurk_ipa_fold_scalars_dev": (_i, [_i, _vp, _sz, _vp, _vp, _i, _vp]),
     "lurk_ipa_fold_bases_dev": (_i, [_i, _vp, _sz, _vp, _vp, _i, _vp]),
     "lurk_ipa_prove_dev": (_i, [_i, _vp, _vp, _vp, _vp, _i, CHALLENGE_FN, _vp, _vp, _vp, _vp, _vp, _i, _vp]),

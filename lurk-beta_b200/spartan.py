@@ -99,6 +99,17 @@ def inner_product(field_id, d_a_ptr, d_b_ptr, n, stream=0):
     return int.from_bytes(out.tobytes(), "little")
 
 
+def poly_combine(field_id, polys, coeffs, d_out_ptr, out_len, stream=0):
+    """PolyEvalWitness::batch_diff_size: out[i] = sum_j coeffs[j] P_j[i], every P_j zero-extended at the end to out_len elements.
+    polys: [(device pointer, length)] of Montgomery elements; coeffs: ints; d_out_ptr: out_len elements, not overlapping any P_j."""
+    n = len(polys)
+    ptrs = (C.c_void_p * n)(*[C.c_void_p(ptr) for ptr, _ in polys])
+    lens = (C.c_size_t * n)(*[int(ln) for _, ln in polys])
+    co = np.concatenate([_fe(c) for c in coeffs]) if coeffs else np.zeros(32, dtype=np.uint8)
+    _capi.check(_capi.lib().lurk_poly_combine_dev(field_id, n, ptrs, lens, _capi.np_ptr(co), C.c_void_p(d_out_ptr), out_len, _capi.FMT_CANONICAL,
+                                                  C.c_void_p(stream)))
+
+
 def ipa_fold_scalars(field_id, d_a_ptr, n, x, y, stream=0):
     _capi.check(_capi.lib().lurk_ipa_fold_scalars_dev(field_id, C.c_void_p(d_a_ptr), n, _capi.np_ptr(_fe(x)), _capi.np_ptr(_fe(y)),
                                                       _capi.FMT_CANONICAL, C.c_void_p(stream)))
@@ -291,3 +302,179 @@ class RelaxedR1CSProver:
         eval_W = inner_product(f, d_z.data_ptr(), eq_ry.data_ptr(), nv)
         mark("eval W", t0)
         return dict(outer_rounds=outer_rounds, inner_rounds=inner_rounds, claims=claims, eval_W=eval_W, rx=rx, ry=ry, E_padded=E)
+
+
+# ------------------------------------------------------------------------------------------------ batch_eval_reduce + BatchedRelaxedR1CSSNARK
+def _powers(x, n, p):
+    out = [1]
+    for _ in range(n - 1):
+        out.append(out[-1] * x % p)
+    return out[:n]
+
+
+def _round_challenge(challenge, label, p):
+    return lambda rnd, msg: challenge(label, (rnd, _ints(np.frombuffer(msg, dtype=np.uint8)))) % p
+
+
+def batch_eval_prove(field_id, claims, challenge, open):
+    """Arecibo's batch_eval_reduce (spartan/mod.rs) -- every evaluation claim of a proof reduced to one claim about one joint
+    polynomial, so a circuit needs ONE polynomial-commitment opening.  claims: [(d_P, point, value)], d_P a device tensor of at least
+    2^len(point) Montgomery elements (read, not modified), value = P(point).  With m_j = len(point_j), m = max m_j:
+      sigma = challenge("batch_r", values); a batched quadratic sum-check over (copy of P_j, eq(point_j)), coefficients sigma^j, round
+      challenges challenge("batch", (round, evals)) -> rho (m elements), left_j = P_j(rho[m - m_j:]);
+      gamma = challenge("batch_g", left); P = sum_j gamma^j P_j (zero-extended to 2^m: lurk_poly_combine_dev);
+      v = sum_j gamma^j L0_j left_j with L0_j = prod_{t < m - m_j} (1 - rho_t)  (= P(rho));  opening = open(P, rho, v).
+    The verifier's joint commitment is sum_j gamma^j comm_j: zero-extension leaves a commitment unchanged."""
+    import torch
+    p = int.from_bytes(field_modulus(field_id), "little")
+    ms = [len(pt) for _, pt, _ in claims]
+    m = max(ms)
+    values = [int(v) % p for _, _, v in claims]
+    sigma = challenge("batch_r", values) % p
+    work = []
+    for (d_P, pt, _), mj in zip(claims, ms):
+        P = d_P[:(1 << mj) * 32].clone()
+        eq = torch.empty_like(P)
+        eq_evals(field_id, [int(x) % p for x in pt], eq.data_ptr())
+        work.append(([P.data_ptr(), eq.data_ptr()], mj, (P, eq)))
+    rounds, rho, fin = sumcheck_prove_batch(field_id, QUAD, [(ptrs, mj) for ptrs, mj, _ in work], values, _powers(sigma, len(claims), p),
+                                            _round_challenge(challenge, "batch", p))
+    del work
+    left = [f[0] for f in fin]
+    gamma = challenge("batch_g", left) % p
+    gp = _powers(gamma, len(claims), p)
+    v = 0
+    for g, mj, lj in zip(gp, ms, left):
+        l0 = 1
+        for t in range(m - mj):
+            l0 = l0 * (1 - rho[t]) % p
+        v = (v + g * l0 * lj) % p
+    joint = torch.empty((1 << m) * 32, dtype=torch.uint8, device="cuda")
+    poly_combine(field_id, [(d_P.data_ptr(), 1 << mj) for (d_P, _, _), mj in zip(claims, ms)], gp, joint.data_ptr(), 1 << m)
+    opening = open(joint, rho, v)
+    return dict(rounds=rounds, rho=rho, values=values, left=left, gamma=gamma, v=v, opening=opening)
+
+
+def fold_running_inputs(prover, ctx):
+    """(padded z, E, u, X) of a NovaFoldContext's running instance for `prover` (same R1CS shape), read where the fold keeps them:
+    W and E stay on the device (LURK_FOLD_BUF_Z1 / E1); only u and X (a few elements) are copied to the host."""
+    from .fold import device_tensor
+    ctx.sync()                                       # the fold's streams are done with the running instance
+    zp, zn = ctx.device_buffer(0, _capi.FOLD_BUF_Z1)
+    ep, en = ctx.device_buffer(0, _capi.FOLD_BUF_E1)
+    z1, e1 = device_tensor(zp, zn), device_tensor(ep, en)
+    tail = z1[prover.n_w * 32:(prover.n_w + 1 + prover.n_x) * 32].clone()
+    _capi.check(_capi.lib().lurk_convert_dev(prover.field, C.c_void_p(tail.data_ptr()), tail.numel() // 32, _capi.FMT_CANONICAL,
+                                             C.c_void_p(tail.data_ptr()), None))
+    ux = _ints(tail.cpu().numpy())
+    return prover.pad_z(z1, ux[0], ux[1:]), e1, ux[0], ux[1:]
+
+
+class BatchedRelaxedR1CSProver:
+    """Control flow of Arecibo's spartan::batched::BatchedRelaxedR1CSSNARK::prove (SuperNova's `compress`, reference
+    src/proof/supernova.rs:110,293-317): the running instances of ALL circuits of an NIVC proof in one argument.  One
+    RelaxedR1CSProver per circuit supplies the device-resident matrices, their transposes and pad_z.  Instance i joins every batched
+    sum-check late and uses the suffix of each shared challenge vector: r_x_i = r_x[s_max - s_i:], r_y_i = r_y[t_max - t_i:]."""
+
+    def __init__(self, provers):
+        self.provers = list(provers)
+        self.field = self.provers[0].field
+        self.p = self.provers[0].p
+        if any(pr.field != self.field for pr in self.provers):
+            raise ValueError("all instances of a batched proof live in one field")
+
+    def prove(self, inputs, challenge, open=None, timings=None):
+        """inputs: per instance (d_z, d_E, u, X) -- padded z (RelaxedR1CSProver.pad_z or fold_running_inputs) and `rows` Montgomery
+        elements of E, device tensors.  Transcript (challenge(label, data) -> int):
+          rho = challenge("outer_r", [(u_i, X_i)]); tau_t = challenge("tau", t), t < s_max; batched cubic sum-check of
+          eq(tau_i) (Az_i Bz_i - (u_i Cz_i + E_i)), claims 0, coefficients rho^i, rounds challenge("outer", ...) -> r_x;
+          claims_i = (Az_i, Bz_i, Cz_i, E_i) at r_x_i; r = challenge("inner_r", claims); batched quadratic sum-check of
+          (A_i + r B_i + r^2 C_i)(r_x_i, .) z_i, claims Az + r Bz + r^2 Cz, coefficients (r^3)^i, rounds challenge("inner", ...) -> r_y;
+          eval_W_i = W_i(r_y_i[1:]).
+        Then, if `open` is given, batch_eval_prove over (W_i, r_y_i[1:], eval_W_i) for every i followed by (E_i, r_x_i, E_i(r_x_i))
+        and the one opening open(d_P, point, value).  Returns the transcript; `eval_claims` are the 2k claims that were reduced."""
+        import time
+        import torch
+        f, p, k = self.field, self.p, len(self.provers)
+        t = time.perf_counter
+
+        def mark(name, t0):
+            if timings is not None:
+                torch.cuda.synchronize()
+                timings[name] = timings.get(name, 0.0) + (t() - t0) * 1e3
+
+        def dev(n):
+            return torch.zeros(n * 32, dtype=torch.uint8, device="cuda")
+        s = [pr.log_rows for pr in self.provers]
+        tv = [pr.num_vars.bit_length() for pr in self.provers]         # log2(2 num_vars)
+        s_max, t_max = max(s), max(tv)
+        t0 = t()
+        prods, Es = [], []
+        for pr, (d_z, d_E, u, _) in zip(self.provers, inputs):
+            Az, Bz, Cz = dev(1 << pr.log_rows), dev(1 << pr.log_rows), dev(1 << pr.log_rows)
+            for M, y in zip(pr.M, (Az, Bz, Cz)):
+                M.mv(f, d_z.data_ptr(), y.data_ptr())
+            E = dev(1 << pr.log_rows)
+            E[:pr.rows * 32] = d_E[:pr.rows * 32]
+            uCzE = torch.empty_like(E)
+            pr._axpy(E, Cz, u, uCzE)
+            prods.append((Az, Bz, Cz, uCzE))
+            Es.append(E)
+        mark("multiply_vec + u Cz + E", t0)
+        t0 = t()
+        rho = challenge("outer_r", [(int(u) % p, [int(x) % p for x in X]) for _, _, u, X in inputs]) % p
+        tau = [challenge("tau", i) % p for i in range(s_max)]
+        work = []
+        for si, (Az, Bz, _, uCzE) in zip(s, prods):
+            eq_tau = torch.empty_like(Az)
+            eq_evals(f, tau[s_max - si:], eq_tau.data_ptr())
+            work.append(([eq_tau, Az.clone(), Bz.clone(), uCzE], si))
+        outer_rounds, rx, fin = sumcheck_prove_batch(f, CUBIC, [([x.data_ptr() for x in w], si) for w, si in work], [0] * k,
+                                                     _powers(rho, k, p), _round_challenge(challenge, "outer", p))
+        del work
+        mark("outer sum-check", t0)
+        t0 = t()
+        eq_rx, claims = [], []
+        for i, (si, (_, _, Cz, _), E) in enumerate(zip(s, prods, Es)):
+            e = torch.empty_like(E)
+            eq_evals(f, rx[s_max - si:], e.data_ptr())
+            eq_rx.append(e)
+            claims.append((fin[i][1], fin[i][2], inner_product(f, Cz.data_ptr(), e.data_ptr(), 1 << si), inner_product(f, E.data_ptr(), e.data_ptr(), 1 << si)))
+        del prods
+        mark("claims at rx", t0)
+        t0 = t()
+        r = challenge("inner_r", claims) % p
+        abcs = []
+        for pr, e in zip(self.provers, eq_rx):
+            ys = [torch.empty(2 * pr.num_vars * 32, dtype=torch.uint8, device="cuda") for _ in range(3)]
+            for M, y in zip(pr.MT, ys):
+                M.mv(f, e.data_ptr(), y.data_ptr())
+            abc = torch.empty_like(ys[0])
+            pr._axpy(ys[0], ys[1], r, abc)
+            pr._axpy(abc, ys[2], r * r % p, abc)
+            abcs.append(abc)
+        del eq_rx
+        mark("eval table (transposed SpMV)", t0)
+        t0 = t()
+        joints = [(c[0] + r * c[1] + r * r * c[2]) % p for c in claims]
+        zcs = [d_z[:2 * pr.num_vars * 32].clone() for pr, (d_z, _, _, _) in zip(self.provers, inputs)]
+        inner_rounds, ry, _ = sumcheck_prove_batch(f, QUAD, [([abc.data_ptr(), zc.data_ptr()], ti) for abc, zc, ti in zip(abcs, zcs, tv)], joints,
+                                                   _powers(r * r * r % p, k, p), _round_challenge(challenge, "inner", p))
+        del abcs, zcs
+        mark("inner sum-check", t0)
+        t0 = t()
+        eval_W = []
+        for pr, ti, (d_z, _, _, _) in zip(self.provers, tv, inputs):
+            eq_ry = torch.empty(pr.num_vars * 32, dtype=torch.uint8, device="cuda")
+            eq_evals(f, ry[t_max - ti + 1:], eq_ry.data_ptr())
+            eval_W.append(inner_product(f, d_z.data_ptr(), eq_ry.data_ptr(), pr.num_vars))
+        mark("eval W", t0)
+        eval_claims = ([(d_z, ry[t_max - ti + 1:], ew) for (d_z, _, _, _), ti, ew in zip(inputs, tv, eval_W)]
+                       + [(E, rx[s_max - si:], c[3]) for E, si, c in zip(Es, s, claims)])
+        out = dict(outer_rounds=outer_rounds, inner_rounds=inner_rounds, claims=claims, eval_W=eval_W, rx=rx, ry=ry, E_padded=Es,
+                   eval_claims=eval_claims)
+        if open is not None:
+            t0 = t()
+            out["batch"] = batch_eval_prove(f, eval_claims, challenge, open)
+            mark("batch_eval_reduce + opening", t0)
+        return out
